@@ -2,7 +2,7 @@
 """bench.py -- X-UNet DDPM training throughput (BASELINE.json metric: train images/sec) on N B200s.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload small64|small128|full128|full64]
-                    [--batch B] [--dtype bf16|fp32] [--no-full128] [--sampler-steps 256]
+                    [--batch B] [--dtype bf16|fp32] [--no-full128] [--sampler-steps 256] [--dump-outputs DIR]
 
 One "step" = one optimisation step (pinned H2D staging -> forward -> backward -> [bucketed NCCL all-reduce, overlapped
 with the backward] -> Adam) on a synthetic SRN-shaped batch of B (source,target) pairs PER GPU (weak scaling).
@@ -21,6 +21,14 @@ Printed JSON (rank 0, one line):
              all-reduce time of the 1.755 GB gradient bucket and how much of it the backward hides; at N=1 also the
              256-step CFG sampler of the full model at 128x128 (views/s at 1 view and at 4 views in flight)
 --impl reference times the CPU oracle alone with the same metric/unit/config (rank 0 only).
+--dump-outputs DIR writes what the last timed device-resident step handed its caller, as float32 .npy files (rank 0): loss,
+the updated params / adam_mu / adam_nu and that step's grads (flat, in the library's parameter order), and e2e_losses (the
+loss of every timed end-to-end step).  The inputs are seeded, so two builds run with the same arguments can be compared
+output for output.  Flat buffers longer than DUMP_MAX_ELEMS (the full model's) are reduced to a fixed, seeded sample of
+DUMP_MAX_ELEMS indices, the same for all four.  The outputs are not bit-reproducible: fp32 atomic reductions differ in the last
+bits from run to run, and bf16 training amplifies that step by step (two runs of one build with the default arguments, 35
+steps, B200 at 1000 W: loss 3e-4, params 1e-2, grads 2e-2 relative L2 apart), so judge a difference between builds against
+the spread of two runs of the same build.
 """
 from __future__ import annotations
 
@@ -47,6 +55,7 @@ WORKLOADS = {
     'full64': ('full', 64, 4, 881_256_824_832),
 }
 METRIC, UNIT = 'xunet_train_images_per_sec', 'images/s'
+DUMP_MAX_ELEMS = 3_000_000      # per flat buffer: 4 buffers x 12 MB stay under 64 MB (the small model's 1.05 M fit whole)
 
 
 _T0 = time.perf_counter()
@@ -428,6 +437,24 @@ class TrainBench:
             self.dev_step(i, step)
         return self.timed(lambda i: self.dev_step(i, step), K)
 
+    def outputs(self):
+        """Host copies of what the last step handed its caller (see --dump-outputs); call it before the next step."""
+        torch = self.torch
+        torch.cuda.synchronize(self.dev)
+        s = self.state
+        flat = {'params': s.params.flat, 'grads': self.eng.grads, 'adam_mu': s.opt_state.mu, 'adam_nu': s.opt_state.nu}
+        n = s.params.flat.numel()
+        idx = None
+        if n > DUMP_MAX_ELEMS:
+            # one seeded index from each of DUMP_MAX_ELEMS equal strides: the same sample at every run, spread over all leaves
+            stride = n // DUMP_MAX_ELEMS
+            pick = np.arange(DUMP_MAX_ELEMS) * stride + np.random.RandomState(0).randint(0, stride, DUMP_MAX_ELEMS)
+            idx = torch.from_numpy(pick).to(self.dev)
+        out = {'loss': self.eng.loss[0].float().cpu().numpy()}
+        for k, v in flat.items():
+            out[k] = (v if idx is None else v.index_select(0, idx)).float().cpu().numpy()
+        return out
+
     def run_e2e(self, K):
         """host numpy inputs through the public API; the loss of every step is read back device->host inside the timed
         region, asynchronously into pinned memory (a real loop logs step i-1 while step i runs); the final synchronize of
@@ -474,7 +501,7 @@ def bench_full128(P, xdist, args, dev, peaks, rank, world):
     import torch
     preset, S, B, fwd_flops = WORKLOADS['full128']
     B = args.full_batch or B
-    K, W = max(3, min(args.steps, args.full_steps)), 3
+    K, W = max(1, min(args.steps, args.full_steps)), 3
     t0 = time.perf_counter()
     progress(f'full128: building the 439 M-parameter model, per-GPU batch {B}')
     tb = TrainBench(P, xdist, preset, S, B, 'bf16', dev, init_on_device=True, n_host=2)
@@ -542,7 +569,12 @@ def main():
     ap.add_argument('--full-batch', type=int, default=0, help='per-GPU batch of the full128 sub-record (default 4)')
     ap.add_argument('--full-steps', type=int, default=8, help='timed steps of the full128 sub-record (<= --steps)')
     ap.add_argument('--ref-budget-s', type=float, default=200.0, help='wall-clock budget of --impl reference')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the outputs of the last timed step to DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs writes the outputs of the b200 path only')
     preset, S, B0, fwd_flops = WORKLOADS[args.workload]
     B = args.batch or B0
     if args.impl == 'reference':
@@ -568,8 +600,15 @@ def main():
         clocks.start()
     # ---- value: inputs resident in HBM; e2e: host numpy inputs through the public API, loss read back every step -------
     t_dev = tb.run_device(args.warmup, args.steps)
+    dumped = tb.outputs() if args.dump_outputs and rank == 0 else None
     progress(f'{args.workload}: {t_dev / args.steps * 1e3:.3f} ms/step device-resident; timing end-to-end')
     t_e2e, h2d, losses = tb.run_e2e(args.steps)
+    if dumped is not None:
+        dumped['e2e_losses'] = np.asarray(losses, dtype=np.float32)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in dumped.items():
+            np.save(os.path.join(args.dump_outputs, name + '.npy'), arr)
+        progress(f'outputs of the last timed step written to {args.dump_outputs}: {sorted(dumped)}')
     clk = clocks.stop() if rank == 0 else None
     progress(f'{args.workload}: e2e {t_e2e / args.steps * 1e3:.3f} ms/step; kernel counts + roofline candidates')
 
